@@ -49,6 +49,8 @@ def parse_args():
                     help="no torchrun: ONE process, one context over --gpus N devices (b200z_create_multi), the whole --size-mib input through the host-pointer calls "
                          "(strong scaling: what one ICompressCoder::Code() call gets from the box)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (compressed stream, decompressed "
+                                                          "bytes) to DIR as .npy files, for comparing two builds output for output")
     return ap.parse_args()
 
 
@@ -358,6 +360,24 @@ def many_files_7z(pkg, codec, n_files=100_000, file_bytes=65536, cpu_files=4000,
     return rec
 
 
+def dump_outputs(out_dir, d_comp, csize, d_back, prop=None, sample=4 << 20, chunk=1 << 20):
+    """What one step of the timed path returned, as float32 / float64 .npy files in out_dir (32 MB for the default 4 GiB):
+    compressed_size (and lzma2_prop), a seeded sample of `sample` bytes of the compressed stream and of the decompressed output
+    (the same positions in every run with the same arguments), and the sum of every `chunk` bytes of both, so that a difference
+    anywhere shows."""
+    import numpy as np, torch
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "compressed_size.npy"), np.array([csize], dtype=np.float64))
+    if prop is not None:
+        np.save(os.path.join(out_dir, "lzma2_prop.npy"), np.array([prop], dtype=np.float64))
+    for name, t in (("compressed", d_comp[:csize]), ("decompressed", d_back)):
+        n = t.numel()
+        idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, sample), replace=False))
+        np.save(os.path.join(out_dir, f"{name}_sample.npy"), t[torch.from_numpy(idx).to(t.device)].cpu().numpy().astype(np.float32))
+        sums = torch.stack([t[i:i + chunk].sum(dtype=torch.int64) for i in range(0, n, chunk)]) if n else torch.zeros(0, dtype=torch.int64)
+        np.save(os.path.join(out_dir, f"{name}_chunk_sums.npy"), sums.cpu().numpy().astype(np.float64))
+
+
 def bind_to_gpu_numa_node(index):
     """Run this rank on the cores of the NUMA node its GPU hangs off, BEFORE any pinned buffer is allocated (first touch then places the
     staging memory next to the GPU's PCIe root: 8 ranks x 12 GB of H2D + D2H per step otherwise cross the socket link for half the GPUs).
@@ -464,11 +484,14 @@ def main():
     d_comp = torch.empty(bound, dtype=torch.uint8, device="cuda")
     d_back = torch.empty(unit_bytes, dtype=torch.uint8, device="cuda")
 
+    last = {}
+
     def step_device():
         if lz:
             t0 = time.perf_counter(); c, prop = codec.lzma2_compress_device(d_in.data_ptr(), unit_bytes, d_comp.data_ptr(), bound); t1 = time.perf_counter()
             n = codec.lzma2_decompress_device(d_comp.data_ptr(), c, prop, d_back.data_ptr(), unit_bytes); t2 = time.perf_counter()
             assert n == unit_bytes
+            last["prop"] = prop
             return c, t1 - t0, t2 - t1
         t0 = time.perf_counter(); c = codec.compress_device(d_in.data_ptr(), unit_bytes, d_comp.data_ptr(), bound); t1 = time.perf_counter()
         n = codec.decompress_device(d_comp.data_ptr(), c, d_back.data_ptr(), unit_bytes); t2 = time.perf_counter()
@@ -485,10 +508,12 @@ def main():
     barrier(); T0 = time.perf_counter()
     t_enc = t_dec = 0.0
     for _ in range(a.steps):
-        _, te, td = step_device(); t_enc += te; t_dec += td
+        csize, te, td = step_device(); t_enc += te; t_dec += td
     barrier(); T1 = time.perf_counter()
     clocks = sampler.stop(T0, T1)
     elapsed = T1 - T0
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, d_comp, csize, d_back, last.get("prop"))
     stats = {k: codec.stat(v) for k, v in dict(match_ms=1, entropy_ms=2, assemble_ms=3, dec_prepass_ms=9, dec_entropy_ms=4, dec_exec_ms=5, launches=6, parse_ms=10).items()}
     if dist:
         t = torch.tensor([elapsed, t_enc, t_dec], device="cuda", dtype=torch.float64)

@@ -1,12 +1,62 @@
 """Test-side access to the checker libraries: oracle/liboracle.so (our C restatement) and
-oracle/_ref/libref_zstd.so (the unmodified reference, compiled by oracle/Makefile)."""
+oracle/_ref/libref_zstd.so (the unmodified reference, compiled by oracle/Makefile), and the recorded answers of the
+reference (tests/golden/reference_answers.json) that stand in for it where it is not built."""
 import ctypes
+import hashlib
+import json
 import os
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 MAXSEQ = 32768
+ANSWERS = os.path.join(ROOT, "tests", "golden", "reference_answers.json")
+
+
+def digest(data) -> str:
+    """short content digest of bytes (what the recorded answers hold instead of the reference's output)"""
+    return hashlib.sha256(bytes(data)).hexdigest()[:16]
+
+
+_answers = None
+
+
+def _tuples(v):
+    return tuple(_tuples(x) for x in v) if isinstance(v, (list, tuple)) else v
+
+
+def reference_answer(question, parts, ask, built):
+    """The reference's answer to `question` about the inputs `parts` (bytes, numbers, strings).
+
+    Where the reference library is `built`, `ask()` computes it (a JSON value: digests, sizes, flags) and it must equal the answer
+    recorded for the same inputs; with B2Z_RECORD_REFERENCE=1 new answers are added to tests/golden/reference_answers.json.
+    Elsewhere the recorded answer is returned, so a build without the reference is still checked against it -- an input that
+    was never put to the reference (our encoder's output changed, say) fails until it is recorded again where the reference is built."""
+    global _answers
+    if _answers is None:
+        _answers = json.load(open(ANSWERS)) if os.path.exists(ANSWERS) else {}
+    h = hashlib.sha256(question.encode())
+    for p in parts:
+        h.update(b"\0" + (bytes(p) if isinstance(p, (bytes, bytearray, memoryview)) else repr(p).encode()))
+    key = f"{question}:{h.hexdigest()[:16]}"
+    if not built:
+        assert key in _answers, f"no recorded answer of the reference for {key}: record it with B2Z_RECORD_REFERENCE=1 where oracle/_ref is built"
+        return _tuples(_answers[key])
+    got = json.loads(json.dumps(ask()))
+    if key in _answers:
+        assert _answers[key] == got, (key, _answers[key], got)
+    elif os.environ.get("B2Z_RECORD_REFERENCE") == "1":
+        _answers[key] = got
+        import fcntl
+        with open(ANSWERS, "a+") as f:                              # pytest-xdist workers record side by side
+            fcntl.flock(f, fcntl.LOCK_EX)
+            f.seek(0)
+            text = f.read()
+            table = json.loads(text) if text else {}
+            table[key] = got
+            f.seek(0); f.truncate()
+            json.dump(table, f, indent=0, sort_keys=True)
+    return _tuples(got)
 
 
 def seq_fields(s):
@@ -150,6 +200,25 @@ def ref_decompress(comp, n) -> bytes:
     return dst[:r].tobytes()
 
 
+def ref_zstd_result(comp, n):
+    """digest of what the reference decoder makes of `comp` (at most n bytes), or "error" (recorded where the reference is absent)"""
+    def ask():
+        try:
+            return digest(ref_decompress(comp, n))
+        except ValueError:
+            return "error"
+    return reference_answer("zstd_decode", (comp, n), ask, ref_available())
+
+
+def ref_size(coder, data, *args, **kw):
+    """size of the reference encoder's output for `data` (coder: ref_compress, ref_lzma2_compress or ref_fl2_compress)"""
+    def ask():
+        out = coder(data, *args, **kw)
+        return len(out if isinstance(out, bytes) else out[1])
+    return reference_answer(f"{coder.__name__}_size", (data, args, sorted(kw.items())), ask,
+                            ref_available() if coder is ref_compress else ref_lzma_available())
+
+
 def sample_inputs(pkg, big=False):
     """name -> bytes: the seeded inputs shared by the CPU and GPU tests (edge cases included)."""
     g2 = pkg.corpus.g2
@@ -176,6 +245,10 @@ _ref_lzma = None
 
 def ref_lzma_available():
     return os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libref_lzma.so"))
+
+
+def ref_xz_available():
+    return os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libref_xz.so"))
 
 
 class _LzmaEncProps(ctypes.Structure):      # C/LzmaEnc.h:13-39
@@ -261,6 +334,22 @@ def ref_lzma2_decompress(comp, n, dict_prop):
     return dst[:dl.value].tobytes(), sl.value
 
 
+def ref_lzma2_result(comp, n, dict_prop):
+    """(digest of the output, bytes consumed) of the reference LZMA2 decoder on `comp`, or None where it reports an error"""
+    def ask():
+        try:
+            out, used = ref_lzma2_decompress(comp, n, dict_prop)
+        except ValueError:
+            return None
+        return digest(out), used
+    return reference_answer("lzma2_decode", (comp, n, dict_prop), ask, ref_lzma_available())
+
+
+def lzma2_result(out_used):
+    """(bytes, consumed) of a decoder in the form ref_lzma2_result answers"""
+    return None if out_used is None else (digest(out_used[0]), out_used[1])
+
+
 def oracle_lzma2_compress(data, **kw):
     """sequential statement of the GPU LZMA2 encoder -> (dictProp, raw LZMA2 stream)"""
     O = oracle(); p = enc_params(**kw); src = _np(data)
@@ -283,6 +372,14 @@ def ref_lzma2_decompress_mt(comp, n, dict_prop, threads):
     if rc != 0:
         raise ValueError(f"reference lzma2 MT decoder error {rc}")
     return dst[:out.value].tobytes(), bool(mt.value)
+
+
+def ref_lzma2_mt_result(comp, n, dict_prop, threads):
+    """(digest of the output, ran multithreaded) of the reference's MT decoder path"""
+    def ask():
+        out, mt = ref_lzma2_decompress_mt(comp, n, dict_prop, threads)
+        return digest(out), mt
+    return reference_answer("lzma2_decode_mt", (comp, n, dict_prop, threads), ask, ref_lzma_available())
 
 
 # ---------------------------------------------------------------- host emulation of the kernel sources (tests/cuemu)

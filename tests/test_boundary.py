@@ -60,8 +60,7 @@ def test_icompresscoder_roundtrip(pkg, tmp_path):
     comp = packed.read_bytes()
     assert comp[:4] == b"\x50\x2a\x4d\x18"                            # mcmilk MT size hint in front of the first frame
     assert helpers.oracle_decompress(comp, len(data)) == data
-    if helpers.ref_available():
-        assert helpers.ref_decompress(comp, len(data)) == data
+    assert helpers.ref_zstd_result(comp, len(data)) == helpers.digest(data)
 
 
 def codec_module_lzma2_roundtrip(pkg, tmp_path, method, level, price_parse):
@@ -77,8 +76,7 @@ def codec_module_lzma2_roundtrip(pkg, tmp_path, method, level, price_parse):
     assert out.returncode == 0 and "roundtrip ok" in out.stdout, out.stderr + out.stdout
     comp = packed.read_bytes()
     assert lzma.LZMADecompressor(format=lzma.FORMAT_RAW, filters=[{"id": lzma.FILTER_LZMA2, "dict_size": 1 << 20}]).decompress(comp) == data
-    if helpers.ref_lzma_available():
-        assert helpers.ref_lzma2_decompress(comp, len(data), 16) == (data, len(comp))
+    assert helpers.ref_lzma2_result(comp, len(data), 16) == (helpers.digest(data), len(comp))
     assert comp == helpers.oracle_lzma2_compress(data, flags=1 | (2 << 8) | (0x10 if price_parse else 0))[1]
 
 

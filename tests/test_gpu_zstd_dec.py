@@ -120,9 +120,8 @@ def test_content_checksums(pkg, inputs):
     comp = c.compress(data)
     assert comp == helpers.oracle_compress(data, flags=3)
     assert c.compress(b"") == helpers.oracle_compress(b"", flags=3)
-    if helpers.ref_available():
-        assert helpers.ref_decompress(comp, len(data)) == data
-        assert helpers.ref_decompress(c.compress(b""), 0) == b""
+    assert helpers.ref_zstd_result(comp, len(data)) == helpers.digest(data)
+    assert helpers.ref_zstd_result(c.compress(b""), 0) == helpers.digest(b"")
     assert c.decompress(comp) == data
     bad = bytearray(comp); bad[-1] ^= 0x40                                   # last byte = part of the last frame's checksum
     with pytest.raises(pkg.B200zError) as e:

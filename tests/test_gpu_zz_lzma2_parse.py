@@ -69,8 +69,7 @@ def test_stream_bit_exact_and_decoders_accept(opt_codec, inputs):
         prop, comp = opt_codec.lzma2_compress(data)
         assert (prop, comp) == helpers.oracle_lzma2_compress(data, flags=1 | (2 << 8) | OPT), name
         assert lzma.LZMADecompressor(format=lzma.FORMAT_RAW, filters=[{"id": lzma.FILTER_LZMA2, "dict_size": _dict_size(prop)}]).decompress(comp) == data, name
-        if helpers.ref_lzma_available():
-            assert helpers.ref_lzma2_decompress(comp, len(data), prop) == (data, len(comp)), name
+        assert helpers.ref_lzma2_result(comp, len(data), prop) == (helpers.digest(data), len(comp)), name
         assert opt_codec.lzma2_decompress(comp, prop) == data, name
 
 
@@ -107,8 +106,7 @@ def test_capped_candidate_is_clipped_at_a_slice_end(pkg):
     prop, comp = c.lzma2_compress(data)
     assert (prop, comp) == helpers.oracle_lzma2_compress(data, frameLog=18, windowLog=18, flags=1 | (1 << 8) | OPT)
     assert c.lzma2_decompress(comp, prop) == data
-    if helpers.ref_lzma_available():
-        assert helpers.ref_lzma2_decompress(comp, len(data), prop)[0] == data
+    assert helpers.ref_lzma2_result(comp, len(data), prop)[0] == helpers.digest(data)
     c.close()
 
 

@@ -46,8 +46,7 @@ def test_frames_bit_exact_and_decoders_accept(zcodec, inputs):
         comp = zcodec.compress(data)
         assert comp == helpers.oracle_compress(data, flags=1 | ZOPT), name
         assert helpers.oracle_decompress(comp, len(data)) == data, name
-        if helpers.ref_available():
-            assert helpers.ref_decompress(comp, len(data)) == data, name
+        assert helpers.ref_zstd_result(comp, len(data)) == helpers.digest(data), name
         assert zcodec.decompress(comp) == data, name
 
 
@@ -80,8 +79,7 @@ def test_codec_module_level_selects_the_parse(pkg, tmp_path):
     assert out.returncode == 0 and "roundtrip ok" in out.stdout, out.stderr + out.stdout
     comp = packed.read_bytes()
     assert comp == helpers.oracle_compress(data, flags=1 | ZOPT)
-    if helpers.ref_available():
-        assert helpers.ref_decompress(comp, len(data)) == data
+    assert helpers.ref_zstd_result(comp, len(data)) == helpers.digest(data)
 
 
 def test_sequence_array_full(pkg, zcodec):
@@ -94,8 +92,7 @@ def test_sequence_array_full(pkg, zcodec):
     comp = zcodec.compress(data)
     assert comp == helpers.oracle_compress(data, flags=1 | ZOPT)
     assert zcodec.decompress(comp) == data
-    if helpers.ref_available():
-        assert helpers.ref_decompress(comp, len(data)) == data
+    assert helpers.ref_zstd_result(comp, len(data)) == helpers.digest(data)
 
 
 def test_capped_candidate_is_clipped_at_a_block_end(pkg, zcodec):

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import helpers as H
-from test_xz_container import _ref_unpack
+from test_xz_container import ref_unpack
 
 pytestmark = pytest.mark.gpu
 
@@ -24,9 +24,8 @@ def test_files_we_write_decode_everywhere(pkg, codec, inputs):
             xz = codec.xz_compress(data, check)
             assert lzma.decompress(xz, format=lzma.FORMAT_XZ) == data, (name, check)
             assert codec.xz_decompress(xz) == data, (name, check)
-        r = _ref_unpack(codec.xz_compress(data, 4), len(data))
-        if r:
-            assert r[0] == 0 and r[1] == data and r[3] != 0, name
+        r = ref_unpack(codec.xz_compress(data, 4), len(data))
+        assert r[0] == 0 and r[1] == H.digest(data) and r[3] != 0, name
     c = pkg.Codec(0, frame_log=18, window_log=18, lzma2_parse=1)     # price-based parse, 256 KiB Blocks
     data = inputs["mixed"] + inputs["g2_1m"]
     xz = c.xz_compress(data)

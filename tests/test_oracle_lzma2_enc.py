@@ -17,8 +17,7 @@ def test_roundtrip_three_decoders(pkg):
         assert prop == 16 and comp[-1] == 0
         assert H.oracle_lzma2_decompress(comp, len(data), prop) == (data, len(comp)), name
         assert lzma.LZMADecompressor(format=lzma.FORMAT_RAW, filters=[{"id": lzma.FILTER_LZMA2, "dict_size": _dict_size(prop)}]).decompress(comp) == data, name
-        if H.ref_lzma_available():
-            assert H.ref_lzma2_decompress(comp, len(data), prop) == (data, len(comp)), name
+        assert H.ref_lzma2_result(comp, len(data), prop) == (H.digest(data), len(comp)), name
 
 
 def test_frame_geometry_and_ratio(pkg):
@@ -41,9 +40,8 @@ def test_frame_geometry_and_ratio(pkg):
     prop, comp = H.oracle_lzma2_compress(data)
     zs = H.oracle_compress(data)
     assert len(comp) < len(zs) * 1.01                             # the same parse (priced for the zstd codes by stage G), range-coded: within 1 % of the zstd frames
-    if H.ref_lzma_available():
-        fl2 = H.ref_fl2_compress(data, 5)[1]
-        assert len(comp) < 1.15 * len(fl2)                        # greedy level-3-class parse in 1 MiB blocks vs FL2 level 5 (optimal parse, 8 MiB dictionary)
+    fl2 = H.ref_size(H.ref_fl2_compress, data, 5)
+    assert len(comp) < 1.15 * fl2                        # greedy level-3-class parse in 1 MiB blocks vs FL2 level 5 (optimal parse, 8 MiB dictionary)
 
 
 def test_incompressible_and_chunk_rollover(pkg):
@@ -54,8 +52,7 @@ def test_incompressible_and_chunk_rollover(pkg):
     mixed = noise[:100_000] + bytes(300_000) + pkg.corpus.g2(500_000).tobytes() + noise[100_000:200_000]
     prop, comp = H.oracle_lzma2_compress(mixed)
     assert H.oracle_lzma2_decompress(comp, len(mixed), prop)[0] == mixed
-    if H.ref_lzma_available():
-        assert H.ref_lzma2_decompress(comp, len(mixed), prop)[0] == mixed
+    assert H.ref_lzma2_result(comp, len(mixed), prop)[0] == H.digest(mixed)
 
 
 def test_state_reset_slices(pkg):
@@ -67,9 +64,8 @@ def test_state_reset_slices(pkg):
         prop, comp = H.oracle_lzma2_compress(data, flags=1 | (sl << 8))
         assert H.oracle_lzma2_decompress(comp, len(data), prop) == (data, len(comp))
         assert lzma.LZMADecompressor(format=lzma.FORMAT_RAW, filters=[{"id": lzma.FILTER_LZMA2, "dict_size": _dict_size(prop)}]).decompress(comp) == data
-        if H.ref_lzma_available():
-            assert H.ref_lzma2_decompress(comp, len(data), prop) == (data, len(comp))
-            assert H.ref_lzma2_decompress_mt(comp, len(data), prop, 4) == (data, True)
+        assert H.ref_lzma2_result(comp, len(data), prop) == (H.digest(data), len(comp))
+        assert H.ref_lzma2_mt_result(comp, len(data), prop, 4) == (H.digest(data), True)
         sizes.append(len(comp))
     assert sizes[0] <= sizes[1] <= sizes[2] <= sizes[3] < sizes[0] * 1.01
 
@@ -81,5 +77,4 @@ def test_large_frames_hit_the_unpack_limit(pkg):
         prop, comp = H.oracle_lzma2_compress(data, frameLog=fl, windowLog=fl, flags=1 | (sl << 8))
         assert prop == (fl - 12) * 2
         assert H.oracle_lzma2_decompress(comp, len(data), prop) == (data, len(comp))
-        if H.ref_lzma_available():
-            assert H.ref_lzma2_decompress(comp, len(data), prop) == (data, len(comp))
+        assert H.ref_lzma2_result(comp, len(data), prop) == (H.digest(data), len(comp))

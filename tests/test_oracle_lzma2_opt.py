@@ -31,8 +31,7 @@ def test_roundtrip_three_decoders(pkg):
         assert prop == 16 and comp[-1] == 0
         assert H.oracle_lzma2_decompress(comp, len(data), prop) == (data, len(comp)), name
         assert lzma.LZMADecompressor(format=lzma.FORMAT_RAW, filters=[{"id": lzma.FILTER_LZMA2, "dict_size": _dict_size(prop)}]).decompress(comp) == data, name
-        if H.ref_lzma_available():
-            assert H.ref_lzma2_decompress(comp, len(data), prop) == (data, len(comp)), name
+        assert H.ref_lzma2_result(comp, len(data), prop) == (H.digest(data), len(comp)), name
 
 
 def test_candidates_are_nearest_previous_occurrences(pkg):
@@ -99,11 +98,10 @@ def test_ratio_moves_towards_the_reference_optimal_parsers(pkg):
     opt22 = len(H.oracle_lzma2_compress(data, flags=1 | (2 << 8) | OPT, frameLog=22, windowLog=22)[1])
     assert opt < 0.955 * greedy                     # measured: 2.54 against 2.40 on G2 text
     assert opt22 < opt1 < opt
-    if H.ref_lzma_available():
-        ref_1m_blocks = len(H.ref_lzma2_compress(data, level=5, dict_size=1 << 20, block_size=1 << 20)[1])    # the reference's optimal parse on the same independent 1 MiB blocks
-        assert opt1 < 1.03 * ref_1m_blocks
-        fl2 = len(H.ref_fl2_compress(data, 5)[1])
-        assert opt22 < 1.06 * fl2
+    ref_1m_blocks = H.ref_size(H.ref_lzma2_compress, data, level=5, dict_size=1 << 20, block_size=1 << 20)    # the reference's optimal parse on the same independent 1 MiB blocks
+    assert opt1 < 1.03 * ref_1m_blocks
+    fl2 = H.ref_size(H.ref_fl2_compress, data, 5)
+    assert opt22 < 1.06 * fl2
 
 
 def test_slices_and_large_frames(pkg):
@@ -112,8 +110,7 @@ def test_slices_and_large_frames(pkg):
         prop, comp = H.oracle_lzma2_compress(data, frameLog=fl, windowLog=fl, flags=1 | (sl << 8) | OPT)
         assert prop == (fl - 12) * 2
         assert H.oracle_lzma2_decompress(comp, len(data), prop) == (data, len(comp))
-        if H.ref_lzma_available():
-            assert H.ref_lzma2_decompress(comp, len(data), prop) == (data, len(comp))
+        assert H.ref_lzma2_result(comp, len(data), prop) == (H.digest(data), len(comp))
 
 
 def test_simulated_model_equals_the_coders_model(pkg):
